@@ -1,226 +1,61 @@
-"""Drop-in proof against the REFERENCE'S OWN classes (SURVEY.md §8b; VERDICT r1 #8, ADVICE r1 medium #1).
+"""Drop-in proof against the REFERENCE'S OWN classes (SURVEY.md §8b).
 
-Runs only where /root/reference exists (the build container; CPU).  tensorflow and hyperopt are absent here, and
-`elliot/recommender/__init__.py:12-25` imports every model eagerly, so a meta-path finder serves permissive stub
-modules for exactly those third-party packages — nothing of the reference itself is stubbed or modified.  In a fresh
-interpreter (so that `elliot_b200.recommender._bases` binds to the reference) the script below checks that
+tests/golden/dropin_reference.json records what the reference framework did with the plugin classes
+(oracle/gen_golden_dropin.py, run with the unmodified reference: elliot's own BaseRecommenderModel, RecMixin, DataSet,
+ModelCoordinator and run_experiment, with `external_models_path` pointing at elliot_b200/external/__init__.py).
+The same case runs here on the stand-alone mirror, in a fresh interpreter with CUDA hidden, and has to agree:
 
-  * `_bases.HOST == "elliot"`: the plugin classes are genuine subclasses of elliot's BaseRecommenderModel ABC with no
-    abstract method left, mixed with elliot's own RecMixin and wrapped by elliot's own `init_charger`;
-  * the plugin module loads through the reference's discovery mechanism (`run.py:67-73`: spec_from_file_location
-    ("external", path) + getattr);
-  * the kernel-side data views (`train_csr_of`, `eval_csr_of`) work on the reference's own DataSet object
-    (`dataset.py:177-245`) and equal what the stand-alone mirror builds from the same frames;
-  * the reference's own `run_experiment` (`run.py:39-148`), given a YAML whose `external_models_path` is
-    elliot_b200/external/__init__.py and whose model key is `external.BPRMF`, gets through its namespace builder, data
-    loader, splitter, logger preparation and plugin discovery and fails only at the CUDA check;
-  * the reference's `ModelCoordinator.single()` (`model_coordinator.py:83-117`) constructs `external.BPRMF` with the
-    reference's keyword contract — the reference's `__init__`/`autoset_params()` fill every `_params_list`
-    attribute — and gets as far as the CUDA check ("needs a CUDA device": there is no CPU fallback);
-  * `name` follows the reference's own shortcut format for the same parameters (compared with the reference BPRMF
-    class's `name` property evaluated on the same attributes).
+  * the plugin classes implement every abstract method of elliot's BaseRecommenderModel ABC;
+  * the kernel-side data views (`train_csr_of`, `eval_csr_of`) and the id order equal what elliot's own DataSet gave
+    for the same frames, both from the mirror DataSet and from an object carrying only the attributes elliot's DataSet
+    has (the models must not rely on mirror-only helpers);
+  * a YAML whose model key is `external.BPRMF` gets through the run_experiment pipeline, plugin discovery included,
+    and fails only at the CUDA check ("needs a CUDA device": there is no CPU fallback), as it did under
+    elliot's ModelCoordinator and run_experiment;
+  * past the availability check the constructor runs the host-side init and dies only in device code;
+  * `autoset_params()` fills the attributes as elliot's did, and `name` follows the reference's own shortcut format
+    (the reference BPRMF class's `name` evaluated on the same attributes).
 """
 import json
 import os
 import subprocess
 import sys
 
-import pytest
-
-REF = "/root/reference"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden", "dropin_reference.json")
 
 SCRIPT = r'''
-import abc, importlib, importlib.abc, importlib.machinery, importlib.util, json, os, sys, tempfile, types
-ROOT, REF = sys.argv[1], sys.argv[2]
-STUBBED = ("tensorflow", "hyperopt", "tensorflow_probability")
-
-class _Meta(abc.ABCMeta):
-    def __getattr__(cls, name):
-        if name.startswith("__"): raise AttributeError(name)
-        return cls
-class Stub(metaclass=_Meta):
-    def __init__(self, *a, **k): pass
-    def __call__(self, *a, **k): return self
-    def __getattr__(self, name):
-        if name.startswith("__"): raise AttributeError(name)
-        return Stub
-class StubModule(types.ModuleType):
-    def __getattr__(self, name):
-        if name.startswith("__"): raise AttributeError(name)
-        return Stub
-class Finder(importlib.abc.MetaPathFinder, importlib.abc.Loader):
-    def find_spec(self, fullname, path, target=None):
-        if fullname.split(".")[0] in STUBBED:
-            return importlib.machinery.ModuleSpec(fullname, self, is_package=True)
-    def create_module(self, spec):
-        m = StubModule(spec.name); m.__path__ = []; return m
-    def exec_module(self, module): pass
-sys.meta_path.insert(0, Finder())
-sys.path.insert(0, REF); sys.path.insert(0, ROOT)
-import logging; logging.disable(logging.CRITICAL)
-from types import SimpleNamespace
-import numpy as np, pandas as pd
-
-out = {}
-from elliot.recommender.base_recommender_model import BaseRecommenderModel as RefBase
-from elliot.recommender.recommender_utils_mixin import RecMixin as RefMixin
-import elliot.dataset.dataset as ref_ds
-from elliot.hyperoptimization.model_coordinator import ModelCoordinator
-from elliot_b200.recommender import _bases
-out["host"] = _bases.HOST
-out["same_base"] = _bases.BaseRecommenderModel is RefBase and _bases.RecMixin is RefMixin
-
-# reference discovery mechanism (run.py:67-73)
-PLUGIN = os.path.join(ROOT, "elliot_b200", "external", "__init__.py")
-spec = importlib.util.spec_from_file_location("external", PLUGIN)
-external = importlib.util.module_from_spec(spec); sys.modules[spec.name] = external; spec.loader.exec_module(external)
-classes = {}
-for name in ("BPRMF", "BPRMF_batch", "MF2020", "MultiVAE", "NeuMF", "MultiDAE", "GMF"):
-    cls = getattr(external, name, None)
-    if cls is None:
-        continue
-    classes[name] = {"subclass": issubclass(cls, RefBase), "mixin": issubclass(cls, RefMixin),
-                     "abstract_left": sorted(cls.__abstractmethods__)}
-out["classes"] = classes
-
-# the reference's own DataSet on a small frame, and the mirror on the same frames
-g = np.random.default_rng(3)
-rows = sorted({(int(10 + 3 * g.integers(60)), int(100 + 7 * g.integers(40))) for _ in range(900)})
-g.shuffle(rows)
-tr = pd.DataFrame({"userId": [r[0] for r in rows[:700]], "itemId": [r[1] for r in rows[:700]], "rating": 1.0})
-keep = set(tr.userId)
-te_rows = [r for r in rows[700:] if r[0] in keep]
-te = pd.DataFrame({"userId": [r[0] for r in te_rows], "itemId": [r[1] for r in te_rows], "rating": 1.0})
-tmp = tempfile.mkdtemp()
-config = SimpleNamespace(config_test=True, align_side_with_train=False, top_k=10, path_output_rec_weight=tmp,
-                         path_output_rec_result=tmp, path_output_rec_performance=tmp,
-                         evaluation=SimpleNamespace(simple_metrics=["nDCG", "HR"], relevance_threshold=0, paired_ttest=False,
-                                                    wilcoxon_test=False, cutoffs=[10]))
-data = ref_ds.DataSet(config, (tr, te), SimpleNamespace())
-out["ref_dataset_has_helper_methods"] = hasattr(data, "train_csr")
-from elliot_b200.dataset import DataSet as Mirror, train_csr_of, eval_csr_of
-mirror = Mirror(config, (tr, te))
-a = train_csr_of(data, "cpu"); b = train_csr_of(mirror, "cpu")
-out["train_csr_equal"] = all(bool((x == y).all()) for x, y in zip(a, b))
-ea, eb = eval_csr_of(data, "test"), eval_csr_of(mirror, "test")
-out["eval_csr_equal"] = all(bool(np.array_equal(x, y)) for x, y in zip(ea, eb))
-out["ids_equal"] = data.users == mirror.users and data.items == mirror.items
-
-# the reference's ModelCoordinator drives external.BPRMF (model_coordinator.py:83-117)
-params = SimpleNamespace(meta=SimpleNamespace(save_recs=False, verbose=False), epochs=2, factors=8, lr=0.05, seed=42,
-                         batch_size=512, user_regularization=0.0025)
-import elliot.utils.logging as elog                          # what run.py:43,66 does before it builds a model
-# the reference's stock elliot/config/logger_config.yml uses a `queue: cfg://objects.queue` handler spec that
-# Python >= 3.12's logging.config rejects (the reference targets 3.6-3.8); it offers `path_logger_config` for a custom
-# one, so the same loggers are declared here with plain console/file handlers.  Nothing of the reference is modified.
-LOGCFG = os.path.join(tmp, "logger_config.yml")
-names = ["recommender", "DataSet", "DataSetLoader", "Evaluator", "namespace", "ModelCoordinator", "prefiltering", "splitter",
-         "result_handler", "EarlyStopping", "__main__"]
-open(LOGCFG, "w").write(
-    "version: 1\nformatters:\n  simple:\n    format: '%(time_filter)-15s: %(levelname)-.1s %(message)s'\n"
-    "filters:\n  time_filter:\n    (): elliot.utils.logging.TimeFilter\n"
-    "handlers:\n  console:\n    class: logging.StreamHandler\n    level: FATAL\n    formatter: simple\n"
-    "    stream: ext://sys.stdout\n    filters: [time_filter]\n"
-    "  file:\n    class: logging.FileHandler\n    level: FATAL\n    filename: !CUSTOM ${log_path_exp}\n    formatter: simple\n"
-    "    filters: [time_filter]\n"
-    "loggers:\n" + "".join(f"  '{n}':\n    level: FATAL\n    handlers: [console, file]\n    propagate: false\n" for n in names)
-    + "root:\n  level: FATAL\n  handlers: [console]\n")
-elog.init(LOGCFG, os.path.join(tmp, "log"))
-elog.prepare_logger("external.BPRMF", os.path.join(tmp, "log"))
-mc = ModelCoordinator([data], config, params, external.BPRMF, 0)
-try:
-    mc.single()
-    out["single"] = "ran"
-except RuntimeError as e:
-    out["single"] = str(e)
-# ... and the reference's own run_experiment drives the whole thing from a YAML file (run.py:39-148): namespace
-# builder, loader + splitter, logger preparation, plugin discovery, ModelCoordinator
-with open(os.path.join(tmp, "dataset.tsv"), "w") as fh:
-    for u, i in rows:
-        fh.write(f"{u}\t{i}\t1.0\t0\n")
-yml = f"""experiment:
-  dataset: dropin
-  data_config:
-    strategy: dataset
-    dataset_path: {tmp}/dataset.tsv
-  splitting:
-    test_splitting:
-      strategy: random_subsampling
-      test_ratio: 0.2
-  top_k: 10
-  evaluation:
-    simple_metrics: [nDCG]
-  path_output_rec_result: {tmp}/recs
-  path_output_rec_weight: {tmp}/weights
-  path_output_rec_performance: {tmp}/perf
-  path_log_folder: {tmp}/log
-  path_logger_config: {LOGCFG}
-  external_models_path: {PLUGIN}
-  models:
-    external.BPRMF:
-      meta:
-        save_recs: False
-      epochs: 2
-      factors: 8
-      lr: 0.05
-"""
-open(os.path.join(tmp, "cfg.yml"), "w").write(yml)
-from elliot.run import run_experiment
-try:
-    run_experiment(os.path.join(tmp, "cfg.yml"))
-    out["run_experiment"] = "ran"
-except RuntimeError as e:
-    out["run_experiment"] = str(e)
-except Exception as e:
-    import traceback
-    out["run_experiment"] = "UNEXPECTED " + type(e).__name__ + ": " + str(e)[:200] + traceback.format_exc()[-800:]
-# constructor contract up to (not including) the device check, through the reference's own init_charger
-import torch
-torch.cuda.is_available = lambda: True                     # let __init__ run past the check; it must then fail INSIDE the device code
-try:
-    external.BPRMF(data=data, config=config, params=SimpleNamespace(**params.__dict__))
-    out["ctor_after_check"] = "constructed"
-except Exception as e:
-    out["ctor_after_check"] = type(e).__name__ + ": " + str(e)[:120]
-# parameters filled by the REFERENCE's autoset_params + the reference's name format
-class Probe(external.BPRMF):
-    def __init__(self): pass
-p = Probe(); RefBase.__init__(p, data, config, SimpleNamespace(**params.__dict__))
-p.logger = logging.getLogger("probe")
-p._params_list = [("_factors", "factors", "f", 10, int, None), ("_learning_rate", "lr", "lr", 0.05, None, None),
-                  ("_bias_regularization", "bias_regularization", "bias_reg", 0, None, None),
-                  ("_user_regularization", "user_regularization", "u_reg", 0.0025, None, None),
-                  ("_positive_item_regularization", "positive_item_regularization", "pos_i_reg", 0.0025, None, None),
-                  ("_negative_item_regularization", "negative_item_regularization", "neg_i_reg", 0.00025, None, None),
-                  ("_update_negative_item_factors", "update_negative_item_factors", "up_neg_i_f", True, None, None),
-                  ("_update_users", "update_users", "up_u", True, None, None), ("_update_items", "update_items", "up_i", True, None, None),
-                  ("_update_bias", "update_bias", "up_b", True, None, None)]
-p.autoset_params()
-out["autoset"] = {"factors": p._factors, "lr": p._learning_rate, "u_reg": p._user_regularization}
-from elliot.recommender.latent_factor_models.BPRMF.BPRMF import BPRMF as RefBPRMF
-out["name_equal"] = external.BPRMF.name.fget(p) == RefBPRMF.name.fget(p)
-out["name"] = external.BPRMF.name.fget(p)
-print("RESULT " + json.dumps(out))
+import json, sys
+sys.path.insert(0, sys.argv[1])
+from oracle.gen_golden_dropin import plugin_facts
+print("RESULT " + json.dumps(plugin_facts()))
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree exists only in the build container")
 def test_plugin_classes_are_driven_by_the_reference_framework():
-    r = subprocess.run([sys.executable, "-c", SCRIPT, ROOT, REF], capture_output=True, text=True, timeout=600,
+    with open(GOLDEN) as fh:
+        ref = json.load(fh)
+    r = subprocess.run([sys.executable, "-c", SCRIPT, ROOT], capture_output=True, text=True, timeout=600,
                        env={**os.environ, "CUDA_VISIBLE_DEVICES": ""})
     line = [l for l in r.stdout.splitlines() if l.startswith("RESULT ")]
     assert line, r.stdout[-2000:] + r.stderr[-3000:]
     out = json.loads(line[-1][7:])
-    assert out["host"] == "elliot" and out["same_base"]
+    assert out["host"] == "standalone"
+    assert out["abstract_methods"] == ref["abstract_methods"]
     assert set(out["classes"]) >= {"BPRMF", "BPRMF_batch", "MF2020", "MultiVAE", "NeuMF"}
+    assert set(out["classes"]) == set(ref["classes"])
     for name, c in out["classes"].items():
         assert c["subclass"] and c["mixin"] and c["abstract_left"] == [], (name, c)
-    assert out["ref_dataset_has_helper_methods"] is False           # the models must not rely on mirror-only methods
-    assert out["train_csr_equal"] and out["eval_csr_equal"] and out["ids_equal"]
-    assert "needs a CUDA device" in out["single"]                    # reached through ModelCoordinator.single()
-    assert "needs a CUDA device" in out["run_experiment"], out["run_experiment"]   # ... and through elliot.run.run_experiment
-    # past the availability check the constructor runs the reference-side init and dies only in device code
-    assert out["ctor_after_check"] != "constructed" and "AttributeError" not in out["ctor_after_check"], out["ctor_after_check"]
-    assert out["autoset"] == {"factors": 8, "lr": 0.05, "u_reg": 0.0025}
-    assert out["name_equal"], out["name"]
+        assert ref["classes"][name] == c, (name, ref["classes"][name])
+    assert ref["dataset_has_helper_methods"] is False
+    for views in (out, out["plain"]):
+        for k in ("train_csr", "eval_csr", "users", "items"):
+            assert views[k] == ref[k], k
+    for k in ("model_coordinator", "run_experiment"):
+        assert "needs a CUDA device" in ref[k], ref[k]
+    assert "needs a CUDA device" in out["construct"], out["construct"]
+    assert out["run_experiment"] == ref["run_experiment"], out["run_experiment"]
+    for facts in (ref, out):
+        assert facts["ctor_after_check"] != "ran" and "AttributeError" not in facts["ctor_after_check"], facts["ctor_after_check"]
+    assert out["autoset"] == ref["autoset"] == {"factors": 8, "lr": 0.05, "u_reg": 0.0025}
+    assert out["name"] == ref["name"], (out["name"], ref["name"])
